@@ -23,6 +23,8 @@ import sys
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -126,11 +128,13 @@ def run_ours(args):
     for i in range(K):
         flush.fill_(i & 0xFF)
         ev[i][0].record()
-        sim.run_round_device()
+        metrics = sim.run_round_device()
         ev[i][1].record()
     barrier()
     launches = small_round.LAUNCH_COUNT["fed_round_small"] - l0
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
+    # what the last timed round handed back, copied before the informational phases below advance the experiment
+    outputs = {"round_metrics": metrics[0].cpu().numpy(), "cluster_models": sim.bank.theta.cpu().numpy()} if args.dump_outputs else {}
 
     # ---- persistent mode (all K rounds inside ONE launch; no flush possible between rounds) — informational
     sim.args.rounds_per_launch = 0
@@ -227,6 +231,10 @@ def run_ours(args):
                                              "reference_as_shipped_rounds_per_s": ref_last.get("value")}
         except (OSError, ValueError):
             pass
+        if outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr.astype(np.float32))
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
@@ -241,7 +249,15 @@ def main():
     ap.add_argument("--no-sleep", dest="no_sleep", action="store_true",
                     help="reference arm only: report the sleep-removed variant as the main value (the as-shipped run always "
                          "carries it as the extra key 'no_sleep')")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed round computed as DIR/<name>.npy (float32): "
+                         "round_metrics [clients, 4] (train correct, train loss sum, test correct, test loss sum) and "
+                         "cluster_models [model slots, parameters]")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         from baseline.run_reference import main as ref_main
         return ref_main(args)

@@ -43,5 +43,5 @@ def test_extra_configs_cover_baseline_configs_2_to_5():
 def test_bench_cli_has_the_driver_contract_flags():
     out = subprocess.run([sys.executable, os.path.join(os.path.dirname(__file__), "..", "bench.py"), "--help"], capture_output=True, text=True,
                          timeout=300).stdout
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--no-sleep"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--no-sleep", "--dump-outputs"):
         assert flag in out, flag
