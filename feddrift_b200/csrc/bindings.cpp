@@ -27,7 +27,8 @@ std::vector<int64_t> fed_round_small(
     c10::optional<Tensor> eval_train_model, c10::optional<Tensor> eval_test_model, c10::optional<Tensor> ens_w,
     c10::optional<Tensor> client_out, c10::optional<Tensor> lr_dev, Tensor metrics, c10::optional<Tensor> timers,
     std::vector<double> fcfg, std::vector<int64_t> icfg, std::vector<int64_t> peer_inbox,
-    c10::optional<Tensor> error_flag, c10::optional<Tensor> counters, std::vector<int64_t> peer_metrics, std::vector<int64_t> host_io) {
+    c10::optional<Tensor> error_flag, c10::optional<Tensor> counters, std::vector<int64_t> peer_metrics, std::vector<int64_t> host_io,
+    c10::optional<Tensor> participants) {
     CHECK_CUDA_F32(X); CHECK_CUDA_I32(Y); CHECK_CUDA_I32(nsamp); CHECK_CUDA_F32(W); CHECK_CUDA_F32(theta); CHECK_CUDA_I32(opt_step);
     CHECK_CUDA_F32(metrics);
     TORCH_CHECK(X.is_contiguous() && Y.is_contiguous() && nsamp.is_contiguous() && W.is_contiguous() && metrics.is_contiguous(),
@@ -44,6 +45,9 @@ std::vector<int64_t> fed_round_small(
     p.opt_m = opt_ptr<float>(opt_m); p.opt_v = opt_ptr<float>(opt_v); p.opt_vmax = opt_ptr<float>(opt_vmax);
     p.opt_step = opt_step.data_ptr<int>();
     p.client_out = opt_ptr<float>(client_out);
+    // [rows, K] int32 client ids per round (validated by ops/small_round.py before the launch)
+    p.participants = opt_ptr<int>(participants);
+    if (p.participants) { p.part_rows = (int)participants->size(0); p.K = (int)participants->size(1); }
     p.lr_ptr = opt_ptr<float>(lr_dev);
     p.metrics = metrics.data_ptr<float>();
     p.timers = (timers.has_value() && timers->defined()) ? reinterpret_cast<long long*>(timers->data_ptr<int64_t>()) : nullptr;
@@ -91,6 +95,14 @@ std::vector<int64_t> fed_round_small(
 
 bool fed_round_small_fits(int64_t kind, int64_t din, int64_t hid, int64_t dout, int64_t C, int64_t M, int64_t t_cur) {
     return fdb::fed_round_small_fits((int)kind, (int)din, (int)hid, (int)dout, (int)C, (int)M, (int)t_cur) != 0;
+}
+
+std::vector<int64_t> fed_round_small_launch_shape(int64_t kind, int64_t din, int64_t hid, int64_t dout, int64_t C, int64_t M,
+                                                  int64_t slots, int64_t cluster, int64_t warps_per_pair) {
+    int smem = 0;
+    const int G = fdb::fed_round_small_launch_shape((int)kind, (int)din, (int)hid, (int)dout, (int)C, (int)M, (int)slots,
+                                                    (int)cluster, (int)warps_per_pair, &smem);
+    return {G, smem};
 }
 
 bool fed_round_small_supported(int64_t kind, int64_t din, int64_t hid, int64_t dout) {
@@ -807,9 +819,16 @@ std::vector<Tensor> lstm_small_grads(Tensor params, Tensor row_off, int64_t off_
 }  // namespace
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
-    m.def("fed_round_small", &fed_round_small);
+    namespace py = pybind11;
+    m.def("fed_round_small", &fed_round_small, py::arg("kind"), py::arg("din"), py::arg("hid"), py::arg("dout"), py::arg("X"),
+          py::arg("Y"), py::arg("nsamp"), py::arg("W"), py::arg("theta"), py::arg("theta_stride"), py::arg("opt_m"), py::arg("opt_v"),
+          py::arg("opt_vmax"), py::arg("opt_step"), py::arg("train_index"), py::arg("train_count"), py::arg("feat_mask"),
+          py::arg("eval_train_model"), py::arg("eval_test_model"), py::arg("ens_w"), py::arg("client_out"), py::arg("lr_dev"),
+          py::arg("metrics"), py::arg("timers"), py::arg("fcfg"), py::arg("icfg"), py::arg("peer_inbox"), py::arg("error_flag"),
+          py::arg("counters"), py::arg("peer_metrics"), py::arg("host_io"), py::arg("participants") = py::none());
     m.def("fed_round_small_supported", &fed_round_small_supported);
     m.def("fed_round_small_fits", &fed_round_small_fits);
+    m.def("fed_round_small_launch_shape", &fed_round_small_launch_shape);
     m.def("mlp_eval_matrix", &mlp_eval_matrix);
     m.def("cluster_aggregate", &cluster_aggregate);
     m.def("cluster_aggregate_opt", &cluster_aggregate_opt);

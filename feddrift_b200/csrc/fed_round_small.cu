@@ -84,7 +84,8 @@ struct BatchSel {
     const int* list; // mode 2: flat sample ids
 };
 
-template <class Net>
+// kPart: a participants table is present (partial participation); the full-participation instance carries none of its code
+template <class Net, bool kPart>
 __global__ void __launch_bounds__(SmallCfg<Net>::kThreads, 1) fed_round_small_kernel(const __grid_constant__ RoundParams p) {
     using Cfg = SmallCfg<Net>;
     constexpr int P = Net::P, IN = Net::kIn, OUT = Net::kOut, HID = Net::kHid;
@@ -97,7 +98,7 @@ __global__ void __launch_bounds__(SmallCfg<Net>::kThreads, 1) fed_round_small_ke
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int C = p.C, M = p.M, S = p.S, t = p.t_cur, B = p.batch_size;
     const int CM = C * M, MP = M * P;
-    const int pairs_per_cta = (CM + G - 1) / G;
+    const int pairs_per_cta = ((kPart ? p.K : C) * M + G - 1) / G;   // must match launch_shape on the host
     const SmemLayout L = make_layout<Net>(M, C, pairs_per_cta);
     float* theta_s = smem + L.theta;
     float* part_s = smem + L.part;
@@ -187,6 +188,10 @@ __global__ void __launch_bounds__(SmallCfg<Net>::kThreads, 1) fed_round_small_ke
 
         // ------------------------------------------------------------------ prep: pair list from W
         if (need_prep) {
+            // partial participation: this round's worker slots → client ids (slot s trains client prow[s]); the table has
+            // one row per round of the time step, rounds past its end wrap around
+            const int* prow = kPart ? p.participants + (size_t)((round0 + r) % p.part_rows) * p.K : nullptr;
+            const int nslots = prow ? p.K : C;
             for (int k = tid; k < CM; k += blockDim.x) {
                 const int c = k / M, m = k % M;
                 float n = 0.f;
@@ -219,29 +224,34 @@ __global__ void __launch_bounds__(SmallCfg<Net>::kThreads, 1) fed_round_small_ke
                 } else {
                     for (int c = 0; c < C; ++c) act |= (p.W[(t * M + m) * C + c] != 0.f);
                 }
-                float tot = 0.f;
-                if (act) for (int c = 0; c < C; ++c) tot += ncm_s[c * M + m];
+                float tot = 0.f;   // aggregation weight total over the clients that train this round
+                if (act) for (int s = 0; s < nslots; ++s) tot += ncm_s[(prow ? prow[s] : s) * M + m];
                 active_s[m] = act;
                 tot_s[m] = tot;
             }
             __syncthreads();
-            if (warp == 0) {  // ordered stream compaction of participating, locally-owned pairs
+            if (warp == 0) {  // ordered stream compaction of participating, locally-owned pairs; keys are slot-major s·M + m
                 int base = 0;
-                for (int k0 = 0; k0 < CM; k0 += 32) {
+                const int SM = nslots * M;
+                for (int k0 = 0; k0 < SM; k0 += 32) {
                     const int k = k0 + lane;
                     bool on = false;
-                    if (k < CM) {
-                        const int c = k / M, m = k % M;
-                        on = active_s[m] && ncm_s[k] > 0.f && (p.world == 1 || (c % p.world) == p.rank);
+                    int c = 0;
+                    if (k < SM) {
+                        const int s = k / M, m = k % M;
+                        c = prow ? prow[s] : s;
+                        on = active_s[m] && ncm_s[c * M + m] > 0.f && (p.world == 1 || (c % p.world) == p.rank);
                     }
                     const unsigned mask = __ballot_sync(0xffffffffu, on);
-                    if (on) pairs_s[base + __popc(mask & ((1u << lane) - 1u))] = k;
+                    // with a table: entry = client << 16 | key (C·M < 2^16: ncm and the pair list alone must fit in 227 KB of
+                    // shared memory)
+                    if (on) pairs_s[base + __popc(mask & ((1u << lane) - 1u))] = kPart ? ((c << 16) | k) : k;
                     base += __popc(mask);
                 }
                 if (lane == 0) misc_s[0] = base;
             }
             __syncthreads();
-            need_prep = (p.recluster_hard != 0);
+            need_prep = (p.recluster_hard != 0) || kPart;
         }
         const int npairs = misc_s[0];
 
@@ -252,22 +262,24 @@ __global__ void __launch_bounds__(SmallCfg<Net>::kThreads, 1) fed_round_small_ke
         // optimizer for the columns it owns and publishes the new local model; two named barriers per step.
         if (gidx < NG) {
         for (int i = crank + G * gidx; i < npairs; i += G * NG) {
-            const int k = pairs_s[i];
-            const int c = k / M, m = k % M;
+            const int e = pairs_s[i];
+            const int k = kPart ? (e & 0xFFFF) : e;       // slot-major: optimizer state / client_out row of worker slot k / M
+            const int c = kPart ? (e >> 16) : k / M;      // the client that slot trains this round (data, batch hash)
+            const int m = k % M;
             const int li = i / G;
             float th[P];
 #pragma unroll
             for (int q = 0; q < P; ++q) th[q] = theta_s[m * P + q];
             float om[COLS], ov[COLS], ovm[COLS];
             int ostep = 0;
-            const size_t obase = (size_t)(c * M + m) * P;
+            const size_t obase = (size_t)k * P;
             double b1pow = 1.0, b2pow = 1.0;
             if (sub == 0) {
 #pragma unroll
                 for (int q = 0; q < COLS; ++q)  // thl = the group's local model; leader lane l owns entries l, l+32, …
                     if (lane + 32 * q < P) thl[lane + 32 * q] = theta_s[m * P + lane + 32 * q];
                 if (p.use_adam) {
-                    ostep = p.opt_step[c * M + m];
+                    ostep = p.opt_step[k];
 #pragma unroll
                     for (int q = 0; q < COLS; ++q) {
                         const int pp = lane + 32 * q;
@@ -396,9 +408,9 @@ __global__ void __launch_bounds__(SmallCfg<Net>::kThreads, 1) fed_round_small_ke
                         const int pp = lane + 32 * q;
                         if (pp < P) { p.opt_m[obase + pp] = om[q]; p.opt_v[obase + pp] = ov[q]; p.opt_vmax[obase + pp] = ovm[q]; }
                     }
-                    if (lane == 0) p.opt_step[c * M + m] = ostep;
+                    if (lane == 0) p.opt_step[k] = ostep;
                 }
-                const float wgt = ncm_s[k] / tot_s[m];
+                const float wgt = ncm_s[kPart ? c * M + m : k] / tot_s[m];
 #pragma unroll
                 for (int q = 0; q < COLS; ++q) {
                     const int pp = lane + 32 * q;
@@ -668,23 +680,38 @@ __global__ void mlp_eval_matrix_kernel(const float* __restrict__ theta, int thet
 }
 
 // ================================================================================ host launchers
+// Cluster size and dynamic shared memory of a launch over `slots` worker slots (C, or K with a participants table).  The
+// per-CTA staging of trained pairs holds ceil(slots·M / G) rows, so a small requested cluster can overflow 227 KB where a
+// larger one fits: the cluster grows (portable sizes, up to 8) until the layout fits.  smem > 227 KB means it never does.
+template <class Net>
+static int launch_shape(int C, int M, int slots, int cluster, int warps_per_pair, int* smem_out) {
+    using Cfg = SmallCfg<Net>;
+    const int rows = slots * M;
+    const int wpp = (warps_per_pair == 4 || warps_per_pair == 2) ? warps_per_pair : 1;
+    const int groups_per_cta = Cfg::kWarps / wpp;
+    int G = cluster;
+    if (G <= 0) {  // auto: enough warp groups for every candidate pair, portable cluster sizes only
+        G = 1;
+        while (G < 8 && G * groups_per_cta < rows) G *= 2;
+    }
+    if (G > 8) G = 8;
+    auto footprint = [&](int g) { return make_layout<Net>(M, C, (rows + g - 1) / g).total * (int)sizeof(float); };
+    int smem = footprint(G);
+    while (smem > 227 * 1024 && G < 8) {
+        G = (2 * G < 8) ? 2 * G : 8;
+        smem = footprint(G);
+    }
+    *smem_out = smem;
+    return G;
+}
+
 template <class Net>
 static int launch_round(const RoundParams& p, int cluster, cudaStream_t stream, SmallLaunchInfo* info) {
     using Cfg = SmallCfg<Net>;
-    const int CM = p.C * p.M;
-    int G = cluster;
-    const int wpp = (p.warps_per_pair == 4 || p.warps_per_pair == 2) ? p.warps_per_pair : 1;
-    const int groups_per_cta = Cfg::kWarps / wpp;
-    if (G <= 0) {  // auto: enough warp groups for every candidate pair, portable cluster sizes only
-        G = 1;
-        while (G < 8 && G * groups_per_cta < CM) G *= 2;
-    }
-    if (G > 8) G = 8;
-    const int pairs_per_cta = (CM + G - 1) / G;
-    const SmemLayout L = make_layout<Net>(p.M, p.C, pairs_per_cta);
-    const int smem = L.total * (int)sizeof(float);
+    int smem = 0;
+    const int G = launch_shape<Net>(p.C, p.M, p.participants ? p.K : p.C, cluster, p.warps_per_pair, &smem);
     if (smem > 227 * 1024) return -2;
-    auto kern = fed_round_small_kernel<Net>;
+    auto kern = p.participants ? fed_round_small_kernel<Net, true> : fed_round_small_kernel<Net, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return -3;
     cudaLaunchConfig_t cfg{};
@@ -708,6 +735,15 @@ int fed_round_small_launch(int kind, int din, int hid, int dout, const RoundPara
                            SmallLaunchInfo* info) {
 #define FDB_CASE(K, I, H, O) \
     if (kind == K && din == I && (K == 0 || hid == H) && dout == O) return launch_round<Mlp<K, I, H, O>>(p, cluster, stream, info);
+    FDB_MLP_SHAPES(FDB_CASE)
+#undef FDB_CASE
+    return -1;
+}
+
+int fed_round_small_launch_shape(int kind, int din, int hid, int dout, int C, int M, int slots, int cluster,
+                                 int warps_per_pair, int* smem) {
+#define FDB_CASE(K, I, H, O) \
+    if (kind == K && din == I && (K == 0 || hid == H) && dout == O) return launch_shape<Mlp<K, I, H, O>>(C, M, slots, cluster, warps_per_pair, smem);
     FDB_MLP_SHAPES(FDB_CASE)
 #undef FDB_CASE
     return -1;

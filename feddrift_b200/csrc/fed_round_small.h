@@ -21,11 +21,16 @@ struct RoundParams {
     const float* ens_w;        // [C, M] or nullptr
     // model / optimizer state
     float* theta;        // [M, theta_stride]
-    float* opt_m;        // [C, M, P]
+    float* opt_m;        // [C, M, P]  (row s·M + m: worker slot s, see participants)
     float* opt_v;
     float* opt_vmax;
     int* opt_step;       // [C, M]
-    float* client_out;   // optional [C, M, P] export of the local models of the LAST round (nullptr = off)
+    float* client_out;   // optional [C, M, P] export of the local models of the LAST round (nullptr = off); slot-indexed
+    // partial participation: row (round0 + r) % part_rows of this table lists the K clients that train in round r;
+    // optimizer state and client_out rows then belong to worker slot s (the s-th listed client), not to client s.
+    // nullptr = every client trains every round (slot == client).
+    const int* participants;   // [part_rows, K] distinct client ids, or nullptr
+    int K, part_rows;
     const float* lr_ptr; // optional device scalar overriding lr
     // outputs
     float* metrics;      // [rounds, C, 4]
@@ -68,6 +73,9 @@ int fed_round_small_launch(int kind, int din, int hid, int dout, const RoundPara
                            SmallLaunchInfo* info);
 int fed_round_small_supported(int kind, int din, int hid, int dout);
 int fed_round_small_fits(int kind, int din, int hid, int dout, int C, int M, int t_cur);
+// cluster size the launcher uses (or -1: shape not instantiated) and its dynamic shared memory in *smem (> 227 KB: no launch)
+int fed_round_small_launch_shape(int kind, int din, int hid, int dout, int C, int M, int slots, int cluster,
+                                 int warps_per_pair, int* smem);
 int mlp_eval_matrix_launch(int kind, int din, int hid, int dout, const float* theta, int theta_stride, int M, const float* X,
                            const int* Y, const int* nsamp, int C, int S, float* correct, float* loss, float* sqerr,
                            cudaStream_t stream);

@@ -14,7 +14,7 @@ Algorithms: ``hard`` / ``hard-r`` (IFCA), ``softmax_α``, ``mmacc_δ`` (FedDrift
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -358,16 +358,23 @@ class SoftClusterState:
         self._log_plurality(t, 0)
 
     def cluster_cfl(self, t: int, round_idx: int, bank: ModelBank, client_params: torch.Tensor,
-                    n: torch.Tensor) -> bool:
-        """``client_params [C, M, P]`` local models, ``n [C, M]`` their sample weights (0 = did not train)."""
+                    n: torch.Tensor, clients: Optional[Sequence[int]] = None) -> bool:
+        """``client_params [C, M, P]`` local models, ``n [C, M]`` their sample weights (0 = did not train).  Under partial
+        participation row s holds the update of client ``clients[s]`` (``None``: row c is client c)."""
         did_split = False
+        row_of = None if clients is None else {int(c): s for s, c in enumerate(clients)}
         in_use = [m for m in range(self.model_num) if (self.W[t][m] > 0).any()]
         for m in in_use:
-            clients = np.nonzero(self.W[t][m])[0]
-            trained = [int(c) for c in clients if float(n[c, m]) != 0]
+            members = np.nonzero(self.W[t][m])[0]
+            if row_of is None:
+                trained = [int(c) for c in members if float(n[c, m]) != 0]
+                rows = trained
+            else:
+                trained = [int(c) for c in members if int(c) in row_of and float(n[row_of[int(c)], m]) != 0]
+                rows = [row_of[c] for c in trained]
             if not trained:
                 continue
-            U = client_params[trained, m, :] - bank.theta[m][None, :]
+            U = client_params[rows, m, :] - bank.theta[m][None, :]
             S, norms = ops.gram_cosine(U)
             max_norm = float(norms.max())
             mean_norm = float(U.mean(dim=0).norm())
@@ -387,7 +394,7 @@ class SoftClusterState:
                         bank.reinit(m)
                         self.W[t][m] = 0.0
                         # g1/g2 index the clients that uploaded an update; idle members stay on m
-                        for c in clients:
+                        for c in members:
                             if int(c) not in trained:
                                 self.W[t][m][c] = 1.0
                         for i in g1:

@@ -28,15 +28,18 @@ CONFIGS = {
 }
 
 
-def measure_config(name: str, device, world: int = 1, rank: int = 0, rounds: Optional[int] = None) -> Dict:
+def measure_config(name: str, device, world: int = 1, rank: int = 0, rounds: Optional[int] = None,
+                   overrides: Optional[Dict] = None) -> Dict:
     """Rounds/s of one named config at time step 1 after a one-round warm-up, device-timed with CUDA events on the launching
     stream (max over ranks is taken by the caller).  Under ``world > 1`` the clients are sharded over the ranks: the fused
-    kernel uses its NVLink peer-inbox mode, the generic executor ``sim.shard_clients`` + the peer aggregation kernel."""
+    kernel uses its NVLink peer-inbox mode, the generic executor ``sim.shard_clients`` + the peer aggregation kernel.
+    ``overrides`` replaces keys of the named config (e.g. ``client_num_per_round``)."""
     import torch
     from ..sim import DriftSim, make_args
     from ..utils.metrics import MetricsSink
     kw = dict(CONFIGS[name])
     kw.update(total_train_iteration=2, epochs=5, lr=0.01, report_client=0)
+    kw.update(overrides or {})
     t0 = time.perf_counter()
     sim = DriftSim(make_args(**kw), device=device, sink=MetricsSink())
     fused = bool(sim.spec is not None and sim.algo.fused_ok())
@@ -68,7 +71,8 @@ def measure_config(name: str, device, world: int = 1, rank: int = 0, rounds: Opt
         ms = float(tt)
     res = {"config": name, "world": world, "rounds": R, "rounds_per_s": R / (ms / 1e3), "ms_per_round": ms / R,
            "setup_s": round(setup, 2), "fused_kernel": fused, "P": sim.bank.P, "clients": sim.C,
-           "last": {k: round(v, 4) for k, v in out.items() if isinstance(v, float)}}
+           "last": {k: round(v, 4) for k, v in out.items() if isinstance(v, float)},
+           "theta_sq_sum": float(sim.bank.theta.detach().double().square().sum())}   # fingerprint of the trained models
     del sim
     torch.cuda.empty_cache()
     return res

@@ -190,6 +190,10 @@ def fed_round_small(st: Dict, rounds: int = 1) -> Dict[str, torch.Tensor]:
     Optional: ``feat_mask [M,din]`` (training inputs only, KUE), ``recluster_hard`` (IFCA per-round argmax
     re-clustering), ``eval_train_model``/``eval_test_model`` [C] int (-1 → argmax_m W[t,m,c]),
     ``ens_mode`` 0|1 (weighted hard vote)|2 (weighted soft vote) with ``ens_w [C,M]`` for the TEST metric.
+    Partial participation: ``participants [rows, K]`` int — round ``round0 + r`` trains only the clients of row
+    ``(round0 + r) % rows``; the s-th of them is worker slot s and uses optimizer-state row ``[s, m]`` (the state follows
+    the slot across rounds, like the reference's per-worker optimizers); each model is the weighted mean of the slots that
+    trained it, in slot order; evaluation still covers all C clients.
     Mutates theta / opt state / W (if recluster) in place; returns ``metrics [rounds, C, 4]`` =
     (train_correct, train_loss_sum, test_correct, test_loss_sum) and ``counts [C, 2]`` = (n_train, n_test).
     """
@@ -206,6 +210,7 @@ def fed_round_small(st: Dict, rounds: int = 1) -> Dict[str, torch.Tensor]:
     feat_mask = st.get("feat_mask")
     ens_mode = int(st.get("ens_mode", 0) or 0)
     Xflat = X.reshape(T1, C, S, -1)
+    part = st.get("participants")
     for r in range(rounds):
         rnd = round0 + r
         cur_lr = float(st["lr"])
@@ -215,8 +220,9 @@ def fed_round_small(st: Dict, rounds: int = 1) -> Dict[str, torch.Tensor]:
         else:
             active = (Wt != 0).any(dim=1)  # [M]
         acc_w = torch.zeros(M, dtype=torch.float64)
-        locals_: Dict[Tuple[int, int], Tuple[torch.Tensor, float]] = {}
-        for c in range(C):
+        locals_: Dict[Tuple[int, int], Tuple[torch.Tensor, float]] = {}   # keyed by (slot, model)
+        sampled = range(C) if part is None else [int(c) for c in part[rnd % part.shape[0]]]
+        for s, c in enumerate(sampled):
             Xc = Xflat[:, c].reshape(T1 * S, -1)
             Yc = Y[:, c].reshape(T1 * S)
             for m in range(M):
@@ -234,21 +240,21 @@ def fed_round_small(st: Dict, rounds: int = 1) -> Dict[str, torch.Tensor]:
                         xb = xb * feat_mask[m]
                     _, g = mlp_loss_grad(p, xb, yb, kind, din, hid, dout)
                     if use_adam:
-                        st["opt_step"][c, m] = adam_amsgrad_update(
-                            p, g, st["opt_m"][c, m], st["opt_v"][c, m], st["opt_vmax"][c, m],
-                            int(st["opt_step"][c, m]), cur_lr, wd)
+                        st["opt_step"][s, m] = adam_amsgrad_update(
+                            p, g, st["opt_m"][s, m], st["opt_v"][s, m], st["opt_vmax"][s, m],
+                            int(st["opt_step"][s, m]), cur_lr, wd)
                     else:
                         p.add_(g, alpha=-cur_lr)
-                locals_[(c, m)] = (p, n_cm)
+                locals_[(s, m)] = (p, n_cm)
                 acc_w[m] += n_cm
         for m in range(M):
             if acc_w[m] <= 0:
                 continue
             tot = np.float32(acc_w[m])
             out = torch.zeros(P, dtype=torch.float32)
-            for c in range(C):
-                if (c, m) in locals_:
-                    p, n_cm = locals_[(c, m)]
+            for s in range(len(sampled)):
+                if (s, m) in locals_:
+                    p, n_cm = locals_[(s, m)]
                     out += p * (np.float32(n_cm) / tot)
             theta[m] = out
         if st.get("recluster_hard", False):

@@ -47,6 +47,21 @@ def _f32(t: Optional[torch.Tensor], dev) -> Optional[torch.Tensor]:
     return t.to(device=dev, dtype=torch.float32).contiguous()
 
 
+def check_participants(table, C: int) -> None:
+    """Raise ``ValueError`` unless ``table`` is a valid partial-participation table for ``C`` clients: int32 ``[rows, K]``
+    with ``1 ≤ K ≤ C``, every id in ``[0, C)`` and the ids of each row distinct."""
+    if not isinstance(table, torch.Tensor) or table.dtype != torch.int32 or table.dim() != 2:
+        raise ValueError("participants must be an int32 tensor of shape [rows, K]")
+    rows, K = table.shape
+    if rows < 1 or not 1 <= K <= C:
+        raise ValueError(f"participants table of shape {tuple(table.shape)}: need at least one row and 1 <= K <= {C}")
+    h = table.detach().cpu()
+    if int(h.min()) < 0 or int(h.max()) >= C:
+        raise ValueError(f"participants table holds client ids outside [0, {C})")
+    if K > 1 and bool((h.sort(dim=1).values.diff(dim=1) == 0).any()):
+        raise ValueError("participants table lists a client twice in one round")
+
+
 def prepare(st: Dict) -> Dict:
     """Build (once per time step) the device views the kernel reads: fp32 X, int32 Y / nsamp / index tables."""
     cache = st.setdefault("_native", {})
@@ -63,6 +78,10 @@ def prepare(st: Dict) -> Dict:
         cache["feat_mask"] = _f32(st.get("feat_mask"), dev)
         cache["eval_train_model"] = _i32(st.get("eval_train_model"), dev)
         cache["eval_test_model"] = _i32(st.get("eval_test_model"), dev)
+        part = st.get("participants")
+        if part is not None:
+            check_participants(part, C)
+            cache["participants"] = part.to(dev).contiguous()
         # launch shape hints: warps per pair from the mini-batch size, cluster size from the active pair count
         B, t = int(st["batch_size"]), int(st["t_cur"])
         bmax = min(B, int(cache["nsamp"].max()))
@@ -78,6 +97,8 @@ def prepare(st: Dict) -> Dict:
             Wc = st["W"][: t + 1].detach().float().cpu()
             active = (Wc[t] != 0).any(dim=1)
             npairs = int(((Wc.sum(0) > 0) & active[:, None]).sum())
+        if part is not None:   # at most K·M pairs train in a round
+            npairs = min(npairs, int(part.shape[1]) * theta.shape[0])
         mg = st.get("multi_gpu")
         if mg:
             npairs = -(-npairs // int(mg["world"]))
@@ -129,7 +150,8 @@ def run_native(st: Dict, rounds: int, metrics_out: Optional[torch.Tensor] = None
         cache["train_index"], cache["train_count"], cache["feat_mask"], cache["eval_train_model"], cache["eval_test_model"],
         ens_w, st.get("client_out"), lr_dev, metrics_out, st.get("timers"), fcfg, icfg,
         list(mg["inbox_ptrs"]) if mg else [], mg.get("error_flag") if mg else None,
-        st.get("counters"), peer_metrics, [int(v) for v in st["host_io"]] if st.get("host_io") else [])
+        st.get("counters"), peer_metrics, [int(v) for v in st["host_io"]] if st.get("host_io") else [],
+        cache.get("participants"))
     if mg:
         mg["flag_base"] = int(mg["flag_base"]) + rounds
     if st.get("counters") is not None:

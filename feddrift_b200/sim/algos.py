@@ -545,14 +545,22 @@ class ClusterFLAlgo(DriftAlgo):
             self.assign = np.asarray(d["clusterfl"]["assign"], dtype=np.int64).copy()
             self.split_done = bool(d["clusterfl"]["split_done"])
 
-    def on_client_updates(self, t: int, client_params: torch.Tensor, n: torch.Tensor) -> bool:
-        """Called by the generic path at the split round with raw local models; returns True if split."""
+    def on_client_updates(self, t: int, client_params: torch.Tensor, n: torch.Tensor,
+                          clients: Optional[List[int]] = None) -> bool:
+        """Called by the generic path at the split round with raw local models; returns True if split.  Under partial
+        participation row s holds the update of client ``clients[s]`` and only those clients can move (``None``: row c is
+        client c)."""
         from ..drift.hclust import complete_linkage_bipartition
         self.split_done = True
-        members = np.nonzero(self.assign == 0)[0]
+        if clients is None:
+            members = np.nonzero(self.assign == 0)[0]
+            rows = members.tolist()
+        else:
+            rows = [s for s, c in enumerate(clients) if self.assign[c] == 0]
+            members = np.asarray([clients[s] for s in rows], dtype=np.int64)
         if len(members) < 2 or self.args.concept_num < 2:
             return False
-        U = client_params[members.tolist(), 0, :] - self.sim.bank.theta[0][None, :]
+        U = client_params[rows, 0, :] - self.sim.bank.theta[0][None, :]
         S, norms = ops.gram_cosine(U)
         self.sim.sink.log({"Max_Norm": float(norms.max()), "Mean_Norm": float(U.mean(0).norm()),
                            "round": self.sim.round_in_step})

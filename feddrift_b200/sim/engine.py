@@ -58,6 +58,17 @@ def make_args(**kw) -> SimpleNamespace:
 from ..ops.small_round import LAUNCH_COUNT as _SMALL_LAUNCHES  # noqa: E402
 
 
+def client_sampling(round_idx: int, client_num_in_total: int, client_num_per_round: int) -> List[int]:
+    """The clients that train in round ``round_idx`` of a time step (``--client_num_per_round`` K of
+    ``--client_num_in_total`` C): all of them when K ≥ C, otherwise the reference's draw
+    ``np.random.seed(round_idx); np.random.choice(range(C), K, replace=False)`` taken from a private ``RandomState`` so that
+    the engine's own random streams are left alone.  The s-th entry is worker slot s."""
+    C, K = int(client_num_in_total), int(client_num_per_round)
+    if K >= C:
+        return list(range(C))
+    return [int(c) for c in np.random.RandomState(round_idx).choice(range(C), K, replace=False)]
+
+
 class DriftSim:
     def __init__(self, args, data: Optional[DriftData] = None, device=None, sink: Optional[MetricsSink] = None,
                  algo=None):
@@ -96,6 +107,13 @@ class DriftSim:
         self.shard_clients = False   # generic path: shard clients over torch.distributed ranks + PeerAggregator
         self.clients = ClientArena(self.C, self.M, self.bank.P, self.device,
                                    adam=(args.client_optimizer != "sgd"))
+        # partial participation: [comm_round, K] sampled client ids per round of a time step (None = every client trains)
+        self.K = min(int(getattr(args, "client_num_per_round", self.C)), self.C)
+        self.participants_table: Optional[torch.Tensor] = None
+        self._participant_rows: List[List[int]] = []
+        if self.K < self.C:
+            self._participant_rows = [client_sampling(r, self.C, self.K) for r in range(max(int(args.comm_round), 1))]
+            self.participants_table = torch.tensor(self._participant_rows, dtype=torch.int32, device=self.device)
         self.timings = {"cluster_s": 0.0, "rounds_s": 0.0}
 
     # ------------------------------------------------------------------ experiment driver
@@ -136,6 +154,19 @@ class DriftSim:
             ckpt.save(self, os.path.join(cdir, f"step_{self.t:04d}.fdck"))
 
     # ------------------------------------------------------------------ rounds
+    def participants(self, r: int) -> List[int]:
+        """Client ids of the worker slots of round ``r`` of the current time step: slot s trains client ``[s]`` and owns row
+        s of the client arena.  The table has ``comm_round`` rows (the reference never runs more rounds in a time step);
+        rounds past that, which only benchmarks and graph replay reach, reuse row ``r % comm_round``."""
+        if self.participants_table is None:
+            return list(range(self.C))
+        return self._participant_rows[r % len(self._participant_rows)]
+
+    def _check_partial_participation(self) -> None:
+        if self.participants_table is not None and (self.multi is not None or getattr(self, "shard_clients", False)):
+            raise ValueError(f"partial participation (client_num_per_round={self.K} < {self.C} clients) is single-GPU only; "
+                             "run with client_num_per_round >= client_num_in_total on several GPUs")
+
     def current_plan(self) -> Dict:
         """The algorithm's training plan for the current time step (built once; sample lists are randomised)."""
         if self._plan is None:
@@ -169,6 +200,8 @@ class DriftSim:
                     self._small[k] = plan[k]
             if self._small["optimizer"] == "sgd":
                 self._small["wd"] = 0.0
+            if self.participants_table is not None:
+                self._small["participants"] = self.participants_table
             if getattr(self, "multi", None) is not None:
                 self._small["multi_gpu"] = self.multi
             if self.device.type == "cuda":  # device-resident round / epoch counters (CUDA-graph replay friendly)
@@ -181,6 +214,7 @@ class DriftSim:
 
     def run_rounds(self, rounds: int) -> Dict:
         """Run ``rounds`` FL rounds of the current time step; returns the last round's aggregate metrics."""
+        self._check_partial_participation()
         t0 = time.perf_counter()
         done, last = 0, {}
         while done < rounds:
@@ -227,6 +261,7 @@ class DriftSim:
     def run_rounds_device(self, n: int) -> torch.Tensor:
         """Launch ``n`` fused rounds and leave the per-round metrics ON DEVICE (no host sync, no logging).
         Returns the device metrics view ``[n, C, 4]``."""
+        self._check_partial_participation()
         st = self._small_state()
         st["round0"] = self.round_in_step
         if self.device.type == "cuda":

@@ -72,7 +72,9 @@ def run_rounds_generic(sim, rounds: int) -> Dict[str, torch.Tensor]:
         bpairs, n_host = [], np.zeros((C, M), dtype=np.float32)
         slots = [] if batched else _stream_slots(sim)    # K side streams: independent (client, model) pairs replay concurrently
         pair_i = 0
-        for c in range(C):
+        # worker slot s trains client sampled[s] in arena row s (slot == client under full participation)
+        sampled = sim.participants(rnd)
+        for s, c in enumerate(sampled):
             if world > 1 and c % world != rank:   # clients are sharded over the ranks (one process per GPU)
                 continue
             xy = _lazy_client_xy(Xc_all, data, c, T1, S)
@@ -83,27 +85,30 @@ def run_rounds_generic(sim, rounds: int) -> Dict[str, torch.Tensor]:
                 if n_cm <= 0:
                     continue
                 if batched:
-                    bpairs.append((c, m, sampler))
-                    n_host[c, m] = n_cm
+                    bpairs.append((s, c, m, sampler))
+                    n_host[s, m] = n_cm
                     continue
                 if slots:
                     with torch.cuda.stream(slots[pair_i % len(slots)]):
-                        cl.params[c, m].copy_(bank.theta[m])
-                        _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, a.wd, feat_mask, pair_i % len(slots))
+                        cl.params[s, m].copy_(bank.theta[m])
+                        _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, a.wd, feat_mask, pair_i % len(slots), s=s)
                 else:
-                    cl.params[c, m].copy_(bank.theta[m])
-                    _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, a.wd, feat_mask)
+                    cl.params[s, m].copy_(bank.theta[m])
+                    _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, a.wd, feat_mask, s=s)
                 pair_i += 1
-                cl.n[c, m] = n_cm
+                cl.n[s, m] = n_cm
         _join_slots(sim, slots)
         if batched:
             if lstm_b:
                 lstm_exec.train_pairs(sim, bpairs, seed, rnd, E, use_adam, lr, a.wd)
             elif not stacked.train_pairs(sim, bpairs, seed, rnd, E, use_adam, lr, a.wd):
-                for (c, m, sampler) in bpairs:            # unequal batch sizes: the per-pair path
-                    cl.params[c, m].copy_(bank.theta[m])
-                    _local_steps(sim, c, m, _lazy_client_xy(Xc_all, data, c, T1, S), sampler, seed, rnd, E, use_adam, lr, a.wd, feat_mask)
+                for (s, c, m, sampler) in bpairs:         # unequal batch sizes: the per-pair path
+                    cl.params[s, m].copy_(bank.theta[m])
+                    _local_steps(sim, c, m, _lazy_client_xy(Xc_all, data, c, T1, S), sampler, seed, rnd, E, use_adam, lr, a.wd, feat_mask,
+                                 s=s)
             cl.n.copy_(torch.from_numpy(n_host), non_blocking=True)
+        # the raw-update hooks address W columns by client id: they get the slot → client list under partial participation
+        uploaded = None if sim.participants_table is None else sampled
         # raw-update hooks (CFL family) may veto the aggregation of this round
         skip = False
         wants_raw = (hasattr(sim.algo, "state") and "cfl" in getattr(sim.algo, "arg", "")) or \
@@ -119,12 +124,12 @@ def run_rounds_generic(sim, rounds: int) -> Dict[str, torch.Tensor]:
             dist.all_reduce(cl.params)
             dist.all_reduce(cl.n)
         if hasattr(sim.algo, "state") and "cfl" in getattr(sim.algo, "arg", ""):
-            skip = sim.algo.state.cluster_cfl(t, rnd + 1, bank, cl.params, cl.n)
+            skip = sim.algo.state.cluster_cfl(t, rnd + 1, bank, cl.params, cl.n, clients=uploaded)
             if skip:
                 plan["W"] = sim.algo.state.weights_tensor(t)
                 st["W"] = plan["W"].cpu()
         if hasattr(sim.algo, "on_client_updates") and not sim.algo.split_done and rnd == sim.algo.split_round:
-            sim.algo.on_client_updates(t, cl.params, cl.n)
+            sim.algo.on_client_updates(t, cl.params, cl.n, clients=uploaded)
         if not skip:
             if world > 1:
                 _peer_aggregate(sim, world, rank)
@@ -336,11 +341,13 @@ def _graphed_step(sim, batch_shape, use_adam, lr, wd, slot: int = 0, steps: int 
     return gs
 
 
-def _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, wd, feat_mask, slot: int = 0):
-    """``xy()`` lazily materialises the client's flattened samples (only the non-indexed paths need that copy)."""
+def _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, wd, feat_mask, slot: int = 0, s: Optional[int] = None):
+    """``xy()`` lazily materialises the client's flattened samples (only the non-indexed paths need that copy).  Client c's
+    data trains arena row ``[s, m]`` (worker slot s; default s = c)."""
     Xc = Yc = None
     bank, cl = sim.bank, sim.clients
-    row = cl.params[c, m]
+    s = c if s is None else s
+    row = cl.params[s, m]
     mlp = bank.mlp
     idxs = []
     for step in range(E):
@@ -355,9 +362,9 @@ def _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, wd, feat_ma
         gidx = (loc // S_) * (C_ * S_) + c * S_ + (loc % S_)
         gs = _graphed_step(sim, (loc.shape[1],) + tuple(sim.data.X.shape[3:]), use_adam, lr, wd, slot, steps=E, indexed=True)
         if gs is not None:
-            gs.load(cl, c, m)
+            gs.load(cl, s, m)
             gs.run_pair(gidx)
-            gs.store(cl, c, m)
+            gs.store(cl, s, m)
             return
     if Xc is None:
         Xc, Yc = xy()
@@ -377,10 +384,10 @@ def _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, wd, feat_ma
             batches.append((xb, Yc[i].long()))
     gs = _graphed_step(sim, batches[0][0].shape, use_adam, lr, wd, slot) if same else None
     if gs is not None:
-        gs.load(cl, c, m)
+        gs.load(cl, s, m)
         for xb, yb in batches:
             gs.run(xb, yb)
-        gs.store(cl, c, m)
+        gs.store(cl, s, m)
         return
     if mlp is None:
         mod = _scratch_module(sim)
@@ -398,8 +405,8 @@ def _local_steps(sim, c, m, xy, sampler, seed, rnd, E, use_adam, lr, wd, feat_ma
             g = _flat_grads(mod, bank, row)
         r2 = row.reshape(1, -1)
         if use_adam:
-            ops.adam_amsgrad_rows_(r2, g.reshape(1, -1), cl.m[c, m].reshape(1, -1), cl.v[c, m].reshape(1, -1),
-                                   cl.vmax[c, m].reshape(1, -1), cl.step[c, m].reshape(1), lr, wd)
+            ops.adam_amsgrad_rows_(r2, g.reshape(1, -1), cl.m[s, m].reshape(1, -1), cl.v[s, m].reshape(1, -1),
+                                   cl.vmax[s, m].reshape(1, -1), cl.step[s, m].reshape(1), lr, wd)
         else:
             ops.sgd_rows_(r2, g.reshape(1, -1), lr, 0.0)
 

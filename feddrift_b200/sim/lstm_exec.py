@@ -59,7 +59,8 @@ def _layout(sim) -> Dict:
 
 
 def train_pairs(sim, pairs: List, seed: int, rnd: int, E: int, use_adam: bool, lr: float, wd: float) -> None:
-    """``pairs``: list of ``(c, m, sampler)``; runs the E local steps of every pair (models start from ``bank.theta[m]``)."""
+    """``pairs``: list of ``(s, c, m, sampler)``; runs the E local steps of every pair (models start from ``bank.theta[m]``) on
+    client c's data in arena row ``[s, m]`` (worker slot s)."""
     bank, cl, dev = sim.bank, sim.clients, sim.device
     C, M, P = sim.C, sim.M, bank.P
     npairs = len(pairs)
@@ -71,7 +72,7 @@ def train_pairs(sim, pairs: List, seed: int, rnd: int, E: int, use_adam: bool, l
     # ---- host: the batch of every (step, pair) from the shared counter-hash RNG; one upload per round
     sel = [[None] * npairs for _ in range(E)]
     bmax = 1
-    for j, (c, m, sampler) in enumerate(pairs):
+    for j, (_, c, m, sampler) in enumerate(pairs):
         for e in range(E):
             h1 = batch_hash(seed, rnd, c, m, e)
             loc = sampler(h1, mix32(h1 ^ 0x68E31DA4)).numpy()
@@ -91,9 +92,9 @@ def train_pairs(sim, pairs: List, seed: int, rnd: int, E: int, use_adam: bool, l
     labels_all = torch.where(valid, Yf[safe], torch.full((), -1, dtype=Yf.dtype, device=dev)).to(torch.int32)            # [E, np, nc·16]
     cnt = valid.sum(-1).clamp(min=1).float()                                                                              # [E, np]
     scale_all = (1.0 / cnt).repeat_interleave(nc, dim=1).contiguous()                                                     # [E, np·nc]
-    rows_h = [c * M + m for c, m, _ in pairs]
+    rows_h = [s * M + m for s, _, m, _ in pairs]
     rows = torch.tensor(rows_h, dtype=torch.int64, device=dev)
-    ms = torch.tensor([m for _, m, _ in pairs], dtype=torch.int64, device=dev)
+    ms = torch.tensor([m for _, _, m, _ in pairs], dtype=torch.int64, device=dev)
     chunk_rows = rows.repeat_interleave(nc)
     chunk_off = (chunk_rows * P).contiguous()
     nch = npairs * nc

@@ -310,7 +310,8 @@ def max_pairs_per_pass(P: int) -> int:
 
 
 def train_pairs(sim, pairs: List, seed: int, rnd: int, E: int, use_adam: bool, lr: float, wd: float) -> bool:
-    """``pairs``: list of ``(c, m, sampler)``.  Runs the E local steps of every pair; returns False (nothing done) when the pairs
+    """``pairs``: list of ``(s, c, m, sampler)``: client c's data trains arena row ``[s, m]`` (worker slot s).  Runs the E local
+    steps of every pair; returns False (nothing done) when the pairs
     draw different batch sizes — the caller then takes the per-pair path.  Large federations are processed in passes of at most
     :func:`max_pairs_per_pass` pairs (equal-sized passes, so at most two staging sets are ever alive)."""
     cap = max_pairs_per_pass(sim.bank.P)
@@ -335,7 +336,7 @@ def _train_pass(sim, pairs: List, seed: int, rnd: int, E: int, use_adam: bool, l
         return True
     S = sim.data.X.shape[2]
     sel = []
-    for (c, m, sampler) in pairs:
+    for (_, c, m, sampler) in pairs:
         row = []
         for e in range(E):
             h1 = batch_hash(seed, rnd, c, m, e)
@@ -353,8 +354,8 @@ def _train_pass(sim, pairs: List, seed: int, rnd: int, E: int, use_adam: bool, l
             stages.clear()
         st = stages[npairs] = _Stage(sim, npairs)
     sim._stack_stage = st
-    rows = torch.tensor([c * M + m for c, m, _ in pairs], dtype=torch.int64, device=dev)
-    ms = torch.tensor([m for _, m, _ in pairs], dtype=torch.int64, device=dev)
+    rows = torch.tensor([s * M + m for s, _, m, _ in pairs], dtype=torch.int64, device=dev)
+    ms = torch.tensor([m for _, _, m, _ in pairs], dtype=torch.int64, device=dev)
     CM = C * M
     torch.index_select(bank.theta, 0, ms, out=st.params)                 # broadcast: every pair starts from its cluster model
     if use_adam:
